@@ -7,7 +7,7 @@ commitment of the LDE rows.  Workload at N=1 = BASELINE.json configs[1]: 234 col
 rate_bits 3, cap_height 4 (2^23 leaves of 234 elements).  Metric = Goldilocks field-elements/s
 (LDE output elements committed per second = B*N / t), whole job.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 N > 1: the SAME commitment is row-block sharded over the ranks (strong scaling): rank g builds leaf rows
@@ -25,6 +25,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
@@ -266,6 +267,59 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step computed, for comparing two builds output for output
+# ------------------------------------------------------------------------------------------------
+DUMP_SEED = 0x0D
+DUMP_LEAF_ROWS = 4096           # sampled Merkle leaves, each with its path
+DUMP_LEAF_BYTES = 24 << 20      # fewer rows when the leaves are wide
+DUMP_COEFFS = 1 << 20           # sampled coefficients
+DUMP_MAX_BYTES = 64 << 20
+
+
+def limbs(words):
+    """Field words as float64, exactly: a trailing axis of 2 holds each word's low and high 32 bits."""
+    w = np.ascontiguousarray(words, dtype=np.uint64)
+    return np.stack([(w & np.uint64(0xFFFFFFFF)).astype(np.float64), (w >> np.uint64(32)).astype(np.float64)], axis=-1)
+
+
+def dump_outputs(out_dir, hnd, cap, fri_result, ctx, dev):
+    """Write what a caller of the timed commitment receives as DIR/<name>.npy (float64):
+    merkle_cap (the whole cap), leaf_rows + merkle_paths (gl_commit_open of leaf_row_index, a fixed seeded sample of
+    leaves), coeffs (the coefficient matrix, column-major, at the flat positions coeff_index, a fixed seeded sample),
+    and with the FRI commit phase fri_caps (one cap per round) and fri_final_poly. Field words go through limbs();
+    the index arrays are plain float64 (exact below 2^53)."""
+    import torch
+
+    from plonky2_b200 import _native as N
+
+    L = N.lib()
+    B, W, log_n = L.gl_commit_num_polys(hnd), L.gl_commit_leaf_width(hnd), L.gl_commit_degree_log(hnd)
+    log_N, h = log_n + L.gl_commit_rate_bits(hnd), L.gl_commit_cap_height(hnd)
+    rng = np.random.default_rng(DUMP_SEED)
+    n_rows = min(1 << log_N, DUMP_LEAF_ROWS, max(1, DUMP_LEAF_BYTES // (16 * W)))
+    rows = np.sort(rng.choice(1 << log_N, n_rows, replace=False)).astype(np.uint64)
+    leaves = np.empty((n_rows, W), dtype=np.uint64)
+    paths = np.empty((n_rows, log_N - h, 4), dtype=np.uint64)
+    N.check(L.gl_commit_open(hnd, N.np_ptr(rows), n_rows, N.np_ptr(leaves), N.np_ptr(paths)), ctx.h)
+    pos = np.sort(rng.choice(B << log_n, min(B << log_n, DUMP_COEFFS), replace=False))
+    coeffs = torch.empty(B << log_n, dtype=torch.int64, device=dev)
+    N.check(L.gl_commit_coeffs(hnd, C.c_void_p(coeffs.data_ptr()), N.MEM_DEVICE), ctx.h)
+    picked = coeffs[torch.from_numpy(pos).to(dev)].cpu().numpy().view(np.uint64)
+    del coeffs
+    arrays = {"merkle_cap": limbs(cap), "leaf_row_index": rows.astype(np.float64), "leaf_rows": limbs(leaves),
+              "merkle_paths": limbs(paths), "coeff_index": pos.astype(np.float64), "coeffs": limbs(picked)}
+    if fri_result is not None:
+        caps, final_poly = fri_result
+        arrays["fri_caps"] = limbs(np.stack([c.hashes for c in caps]))
+        arrays["fri_final_poly"] = limbs(final_poly)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "output dump of %d bytes exceeds %d" % (total, DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+# ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
 def gpu_arm(args, rank, local_rank, world):
@@ -356,7 +410,8 @@ def gpu_arm(args, rank, local_rank, world):
         fri_out = [None]
         fri_spans = []
 
-        def step_device():
+        def step_device(keep=False):
+            """One step; keep=True returns the commitment handle instead of destroying it."""
             if committer is not None:
                 # column-sharded iNTT -> NCCL all-gather of coefficients -> row-block sharded LDE + Merkle
                 hnd = committer.commit(vals, from_host=False)
@@ -375,6 +430,8 @@ def gpu_arm(args, rank, local_rank, world):
                 fri_out[0] = fri_ctx(hnd, cap_full.cpu().numpy())
                 fb.record(stream)
                 fri_spans.append((fa, fb))
+            if keep:
+                return hnd
             L.gl_commit_destroy(hnd)
 
         def sync_all():
@@ -396,8 +453,10 @@ def gpu_arm(args, rank, local_rank, world):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
         marks = []
-        for _ in range(args.steps):
-            step_device()
+        last = None
+        for k in range(args.steps):
+            # with --dump-outputs the last step's commitment outlives the timed window (its free is stream-ordered)
+            last = step_device(keep=bool(args.dump_outputs) and k == args.steps - 1)
             m = torch.cuda.Event(enable_timing=True)
             m.record(stream)
             marks.append(m)
@@ -420,6 +479,9 @@ def gpu_arm(args, rank, local_rank, world):
         if fixture is not None:  # golden cap of this exact workload from the CPU oracle (tests/golden/fullscale_*.json)
             cap_ok = bool(np.array_equal(cap_dev, np.array(fixture["cap"], dtype=np.uint64)))
             assert cap_ok, "rank %d: the gathered Merkle cap differs from the oracle fixture" % rank
+        if last is not None:
+            dump_outputs(args.dump_outputs, last, cap_dev, fri_out[0], ctx, dev)
+            L.gl_commit_destroy(last)
 
         # ---- end to end through the C ABI with HOST buffers (pinned): H2D of the columns + D2H of the cap
         host_vals = torch.empty((B, n), dtype=torch.int64, pin_memory=True)
@@ -662,11 +724,12 @@ def recursion_shape(ctx_device, reps=5):
     # the same sequence through the compiled C++ host layer (include/plonky2_b200.hpp): no Python in the loop
     cpp = None
     try:
-        exe = os.path.join(tempfile.gettempdir(), "gl_prove_latency")
-        subprocess.check_call(["g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), "-o", exe,
-                               os.path.join(ROOT, "tools", "prove_latency.cpp"), "-L" + os.path.join(ROOT, "plonky2_b200"),
-                               "-lplonky2_b200", "-Wl,-rpath," + os.path.join(ROOT, "plonky2_b200")])
-        cpp = json.loads(subprocess.run([exe, "7"], capture_output=True, text=True, timeout=120).stdout.strip().splitlines()[-1])
+        with tempfile.TemporaryDirectory() as tmp:
+            exe = os.path.join(tmp, "gl_prove_latency")
+            subprocess.check_call(["g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), "-o", exe,
+                                   os.path.join(ROOT, "tools", "prove_latency.cpp"), "-L" + os.path.join(ROOT, "plonky2_b200"),
+                                   "-lplonky2_b200", "-Wl,-rpath," + os.path.join(ROOT, "plonky2_b200")])
+            cpp = json.loads(subprocess.run([exe, "7"], capture_output=True, text=True, timeout=120).stdout.strip().splitlines()[-1])
     except Exception as e:
         cpp = {"error": repr(e)}
     return {"cpp_host": cpp,"workload": "recursion-shaped synthetic proof, n=2^14, standard_recursion_config "
@@ -754,8 +817,12 @@ def main():
     ap.add_argument("--ntt-group", type=int, default=0, help="columns per NTT group (0 = library default)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the recursion-shaped prove() timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     ap.add_argument("--plonk-circuit-only", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl b200 on one GPU")
     if args.plonk_circuit_only:   # child mode of the secondary measurement `prove_plonk_circuit`
         try:
             print(json.dumps(plonk_circuit_proof(0)), flush=True)

@@ -137,14 +137,14 @@ def test_fri_proof_serialisation_layout():
     assert b[8 * 8 + 3 * 8] == 2
 
 
-def test_cpp_host_layer_compiles_and_fails_loudly_without_gpu(native, oracle):
+def test_cpp_host_layer_compiles_and_fails_loudly_without_gpu(native, oracle, tmp_path):
     """include/plonky2_b200.hpp (the C++ mirror of the reference's Rust interface) builds against the C ABI;
     without a GPU the program must abort with the library's "no CPU fallback" error, not compute anything."""
     import subprocess
 
     import torch
 
-    exe = "/tmp/gl_host_parity_cpu"
+    exe = str(tmp_path / "gl_host_parity_cpu")
     subprocess.check_call(["g++", "-std=c++17", "-O0", "-Wall", "-I", os.path.join(ROOT, "include"), "-o", exe,
                            os.path.join(ROOT, "tests", "cpp", "host_parity.cpp"),
                            "-L" + os.path.join(ROOT, "plonky2_b200"), "-lplonky2_b200",

@@ -9,11 +9,11 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _build_and_run(src, exe, args=(), defs=()):
+def _build_and_run(tmp_path, src, exe, args=(), defs=()):
     import oracle_lib
 
     oracle_lib.build_oracle()
-    out = os.path.join("/tmp", exe)
+    out = str(tmp_path / exe)
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-DGL_FORCE_32BIT_PATH", *defs, "-o", out,
                            os.path.join(ROOT, "tests", "emu", src), "-L" + os.path.join(ROOT, "oracle"),
                            "-lgl_oracle", "-Wl,-rpath," + os.path.join(ROOT, "oracle"), "-pthread"])
@@ -22,17 +22,17 @@ def _build_and_run(src, exe, args=(), defs=()):
     return r.stdout
 
 
-def test_field_and_poseidon_device_formulation_on_host():
-    assert "EMU OK" in _build_and_run("field_poseidon_emu.cpp", "gl_fp_emu")
+def test_field_and_poseidon_device_formulation_on_host(tmp_path):
+    assert "EMU OK" in _build_and_run(tmp_path, "field_poseidon_emu.cpp", "gl_fp_emu")
 
 
-def test_ntt_tiles_forward_inverse_lde_on_host():
+def test_ntt_tiles_forward_inverse_lde_on_host(tmp_path):
     # log_n 1..13: single-pass (<= 12) and two-pass (13) plans; forward, inverse and leaf-major coset LDE
-    assert "EMU OK" in _build_and_run("ntt_emu.cpp", "gl_ntt_emu", ["13"])
+    assert "EMU OK" in _build_and_run(tmp_path, "ntt_emu.cpp", "gl_ntt_emu", ["13"])
 
 
-def test_poseidon_fp64_pipe_formulation_on_host():
+def test_poseidon_fp64_pipe_formulation_on_host(tmp_path):
     # the FP64 MDS layers and the FP64-resident partial rounds (device default) with IEEE doubles on the CPU:
     # bit-exact vs both oracle forms (fast and naive partial rounds), limb magnitudes stay below 2^51
-    out = _build_and_run("poseidon_f64_emu.cpp", "gl_f64_emu", ["60000"], defs=["-DGL_FP64_ON_HOST"])
+    out = _build_and_run(tmp_path, "poseidon_f64_emu.cpp", "gl_f64_emu", ["60000"], defs=["-DGL_FP64_ON_HOST"])
     assert "POSEIDON F64 EMU OK" in out, out

@@ -599,13 +599,13 @@ def test_profiling_phases_and_launch_count(pb):
     ctx.close()
 
 
-def test_cpp_host_layer_parity(pb):
+def test_cpp_host_layer_parity(pb, tmp_path):
     """The compiled-language host layer (include/plonky2_b200.hpp, mirroring the reference's Rust interface)
     driven by tests/cpp/host_parity.cpp: NTT vs naive evaluation, commitment vs oracle, shape errors,
     byte-identical FriProof accepted by the restated verifier."""
     import subprocess
 
-    exe = "/tmp/gl_host_parity"
+    exe = str(tmp_path / "gl_host_parity")
     subprocess.check_call(["g++", "-std=c++17", "-O1", "-I", os.path.join(ROOT, "include"), "-o", exe,
                            os.path.join(ROOT, "tests", "cpp", "host_parity.cpp"),
                            "-L" + os.path.join(ROOT, "plonky2_b200"), "-lplonky2_b200",

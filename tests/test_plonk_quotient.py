@@ -228,7 +228,7 @@ def test_selector_groups_follow_the_reference_rule():
 
 
 @pytest.mark.parametrize("nc", [1, 3, 4])
-def test_other_challenge_counts_through_the_kernel_source(oracle, nc):
+def test_other_challenge_counts_through_the_kernel_source(oracle, emu_lib, nc):
     """num_challenges = 1, 3, 4 (the kernel's accumulator bound): identity for the oracle, bit-exactness for the program."""
     for shape in (SHAPES[1], SHAPES[6]):
         c = _circuit(shape, num_challenges=nc)
@@ -239,17 +239,18 @@ def test_other_challenge_counts_through_the_kernel_source(oracle, nc):
         zeta = int(synth(0x5A2, (1,))[0])
         want, zh = _vanishing_at(c, cs, w, z, zeta, betas, gammas, alphas, deltas)
         assert all(want[i] == zh * _ev(q[i], zeta) % P_ for i in range(nc))
-        assert np.array_equal(_emu_quotient(oracle, c, cs, w, z, betas, gammas, alphas, deltas), q)
+        assert np.array_equal(_emu_quotient(emu_lib, oracle, c, cs, w, z, betas, gammas, alphas, deltas), q)
 
 
-def _emu_lib():
-    out = "/tmp/libgl_vanishing_emu.so"
+@pytest.fixture(scope="module")
+def emu_lib(tmp_path_factory):
+    out = str(tmp_path_factory.mktemp("emu") / "libgl_vanishing_emu.so")
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-DGL_FORCE_32BIT_PATH", "-shared", "-fPIC", "-o", out,
                            os.path.join(ROOT, "tests", "emu", "vanishing_emu.cpp")])
     return C.CDLL(out)
 
 
-def _emu_quotient(oracle, c, cs, w, z, betas, gammas, alphas, deltas):
+def _emu_quotient(L, oracle, c, cs, w, z, betas, gammas, alphas, deltas):
     """The product's program interpreted by the kernel's per-point source on the host, then coset_ifft."""
     cfg, cd = c.config, c.common
     nc = cfg.num_challenges
@@ -264,7 +265,6 @@ def _emu_quotient(oracle, c, cs, w, z, betas, gammas, alphas, deltas):
     size = c.n << qd_bits
     vals = np.zeros((nc, size), dtype=np.uint64)
     al = np.array(alphas, dtype=np.uint64)
-    L = _emu_lib()
     L.emu_plonk_quotient_values.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
                                             C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p]
     rc = L.emu_plonk_quotient_values(ptrs, strides, 3, cfg.rate_bits, cd.degree_bits, qd_bits, prog, len(prog),
@@ -274,14 +274,14 @@ def _emu_quotient(oracle, c, cs, w, z, betas, gammas, alphas, deltas):
 
 
 @pytest.mark.parametrize("shape", SHAPES + [LOOKUP_SHAPE_64, (135, 80, 8, 3, 6, 20), (135, 80, 8, 3, 7)])
-def test_vanishing_program_through_the_kernel_source_on_host_matches_oracle(oracle, shape):
+def test_vanishing_program_through_the_kernel_source_on_host_matches_oracle(oracle, emu_lib, shape):
     c = _circuit(shape)
     nc = c.config.num_challenges
     betas, gammas, alphas = _challenges(0x540 + shape[0], nc)
     deltas = _deltas(c, 0x541)
     cs, w, z = _oracle_commits(oracle, c, betas, gammas, deltas)
     want = oracle.plonk_quotient(c.oracle_circuit(), cs, w, z, c.public_inputs_hash, betas, gammas, alphas, deltas)
-    assert np.array_equal(_emu_quotient(oracle, c, cs, w, z, betas, gammas, alphas, deltas), want)
+    assert np.array_equal(_emu_quotient(emu_lib, oracle, c, cs, w, z, betas, gammas, alphas, deltas), want)
 
 
 @pytest.mark.parametrize("broken", ["pair", "table"])
