@@ -211,6 +211,8 @@ int gl_lookup_polys(gl_ctx* ctx, const uint64_t* wires, uint32_t log_n, uint32_t
 #define GL_STARK_SUB 4
 #define GL_STARK_MUL 5
 #define GL_STARK_EMIT 6  /* a = value, b = GL_STARK_CONSTRAINT / _TRANSITION / _FIRST_ROW / _LAST_ROW */
+#define GL_STARK_AUX_LOCAL 7 /* a = auxiliary polynomial: local row value (gl_stark_quotient_aux only) */
+#define GL_STARK_AUX_NEXT 8  /* a = auxiliary polynomial: next row value */
 #define GL_STARK_CONSTRAINT 0
 #define GL_STARK_TRANSITION 1
 #define GL_STARK_FIRST_ROW 2
@@ -224,6 +226,51 @@ typedef struct {
 int gl_stark_quotient(gl_ctx* ctx, gl_commit* trace, const gl_stark_instr* program, uint32_t n_instr,
                       const uint64_t* consts, uint32_t n_consts, const uint64_t* alphas, uint32_t n_alphas,
                       uint32_t quotient_degree_factor, uint64_t* out_coeffs);
+/* The same with the auxiliary polynomials (starky/src/prover.rs:488-668 with auxiliary_polys_commitment): GL_STARK_AUX_LOCAL /
+ * GL_STARK_AUX_NEXT read aux's LDE in place with the trace's addressing. aux may be NULL (then this is gl_stark_quotient);
+ * otherwise it has the trace's degree and rate. The logUp constraints (eval_packed_lookups_generic, lookup.rs:804-863) are
+ * ordinary instructions of the program, emitted after the STARK's own; their challenges travel in consts. */
+int gl_stark_quotient_aux(gl_ctx* ctx, gl_commit* trace, gl_commit* aux, const gl_stark_instr* program, uint32_t n_instr,
+                          const uint64_t* consts, uint32_t n_consts, const uint64_t* alphas, uint32_t n_alphas,
+                          uint32_t quotient_degree_factor, uint64_t* out_coeffs);
+
+/* logUp helper columns of a STARK's lookups (lookup_helper_columns / get_helper_cols, starky/src/lookup.rs:579-652,746-789)
+ * for every lookup and every challenge gamma, lookup-major and challenge-minor, as value columns of n = 2^log_n rows:
+ *   ceil(n_looking / chunk) helper columns h_k = sum_{i in chunk k} filter_i / (f_i + gamma),  chunk = max(1, constraint_degree - 1),
+ *   then Z with Z(0) = 0, Z(i+1) = Z(i) + sum_k h_k(i) - m(i) / (t(i) + gamma).
+ * Columns and filters are evaluated like eval_table (lookup.rs:318-329): next-row terms read row (i + 1) mod n. The trace is
+ * n_cols columns, column c at trace + c * col_stride; out = the helper columns, column j at out + j * n. trace and out are both
+ * host (GL_MEM_HOST) or both device (GL_MEM_DEVICE) memory. A zero denominator fails with GL_ERR_DIV_ZERO ("Tried to invert
+ * zero"), where batch_multiplicative_inverse panics. At most GL_LOGUP_MAX_DENOMINATORS = sum over lookups of
+ * (n_looking + 1) * n_challenges per row. */
+typedef struct {
+    uint32_t col, next; /* coeff * trace[col][row], or [row + 1 mod n] if next (Column::linear_combination / next_row_...) */
+    uint64_t coeff;
+} gl_logup_term;
+typedef struct {
+    uint32_t term_begin, n_terms; /* Column<F> (lookup.rs:137-160): terms[term_begin ..+ n_terms] + constant */
+    uint64_t constant;
+} gl_logup_column;
+typedef struct {
+    uint32_t prod_begin, n_prods; /* Filter<F> (lookup.rs:33-45): sum_j col(fc[prod_begin + 2j]) * col(fc[prod_begin + 2j + 1]) */
+    uint32_t sum_begin, n_sums;   /*   + sum_j col(fc[sum_begin + j]),  fc = gl_logup_desc.filter_columns */
+} gl_logup_filter;
+typedef struct {
+    uint32_t looking_begin, n_looking; /* Lookup<F> (lookup.rs:403-416): looking column k = columns[looking_begin + k], */
+    uint32_t table, frequencies;       /*   its filter = filters[looking_begin + k]; table / frequencies: column indices */
+} gl_logup_lookup;
+typedef struct {
+    const gl_logup_term* terms;
+    const gl_logup_column* columns;
+    const uint32_t* filter_columns;
+    const gl_logup_filter* filters; /* as many as columns (entries of table / frequency columns are unused) */
+    const gl_logup_lookup* lookups;
+    uint32_t n_terms, n_columns, n_filter_columns, n_lookups;
+} gl_logup_desc;
+#define GL_LOGUP_MAX_DENOMINATORS 128
+int gl_stark_lookup_helper_columns(gl_ctx* ctx, const uint64_t* trace, size_t col_stride, uint32_t n_cols, uint32_t log_n,
+                                   const gl_logup_desc* desc, const uint64_t* challenges, uint32_t n_challenges,
+                                   uint32_t constraint_degree, uint64_t* out, int mem);
 
 /* compute_quotient_polys of a plonky2 circuit (plonky2/src/plonk/prover.rs:609-815): for every challenge alpha_k the
  * values eval_vanishing_poly_base_batch(x) / Z_H(x) (plonky2/src/plonk/vanishing_poly.rs:167-340) on the coset g<w_size>,

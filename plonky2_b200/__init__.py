@@ -13,8 +13,9 @@ from .fri import (FriBatchInfo, FriConfig, FriInstanceInfo, FriOracleInfo, FriPa
 from .hash import (MerkleCap, MerkleProof, MerkleTree, PoseidonHash, PoseidonPermutation,  # noqa: F401
                    verify_merkle_proof_to_cap)
 from .polynomial_batch import SALT_SIZE, PolynomialBatch  # noqa: F401
-from .proof import OpeningSet, StarkOpeningSet, eval_commitments  # noqa: F401
-from .stark import FibonacciStark, Stark, commit_quotient_polys, compute_quotient_polys  # noqa: F401
+from .proof import OpeningSet, StarkOpeningSet, StarkProof, StarkProofWithPublicInputs, eval_commitments  # noqa: F401
+from .stark import (Column, FibonacciStark, Filter, Lookup, PermutationStark, Stark, StarkConfig,  # noqa: F401
+                    commit_quotient_polys, compute_quotient_polys)
 from . import plonk  # noqa: F401  (plonk.compute_quotient_polys: the plonky2 circuit quotient)
 from .batch_merkle_tree import (BatchMerkleTree, compress_merkle_proofs, decompress_merkle_proofs,  # noqa: F401
                                 verify_batch_merkle_proof_to_cap)

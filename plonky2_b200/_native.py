@@ -26,7 +26,7 @@ EXPORTS = [
     "gl_commit_finish", "gl_commit_shard", "gl_commit_destroy", "gl_commit_num_polys",
     "gl_commit_leaf_width", "gl_commit_degree_log", "gl_commit_rate_bits", "gl_commit_cap_height",
     "gl_commit_cap", "gl_commit_coeffs", "gl_commit_leaves", "gl_commit_digests", "gl_commit_get_lde_values",
-    "gl_commit_open", "gl_commit_eval_ext", "gl_openings", "gl_stark_quotient", "gl_plonk_quotient", "gl_lookup_polys", "gl_commit_dev_lde", "gl_commit_dev_coeffs", "gl_partial_products_and_zs", "gl_poseidon_permute_host",
+    "gl_commit_open", "gl_commit_eval_ext", "gl_openings", "gl_stark_quotient", "gl_stark_quotient_aux", "gl_stark_lookup_helper_columns", "gl_plonk_quotient", "gl_lookup_polys", "gl_commit_dev_lde", "gl_commit_dev_coeffs", "gl_partial_products_and_zs", "gl_poseidon_permute_host",
     "gl_poseidon_permute_many", "gl_poseidon_hash_many", "gl_poseidon_hash_no_pad_many", "gl_poseidon_two_to_one_many", "gl_merkle_build", "gl_merkle_destroy",
     "gl_merkle_cap", "gl_merkle_digests", "gl_merkle_open", "gl_fri_begin", "gl_fri_begin_values", "gl_fri_values_local", "gl_fri_begin_from_coeffs",
     "gl_fri_destroy", "gl_fri_coeffs", "gl_fri_commit_round", "gl_fri_commit_round_sharded", "gl_fri_mix", "gl_fri_fold", "gl_fri_final_poly",
@@ -100,6 +100,9 @@ def lib():
     L.gl_commit_eval_ext.argtypes = [vp, vp, vp]
     L.gl_openings.argtypes = [vp, C.POINTER(vp), u32p, C.c_size_t, vp, C.c_size_t, vp, C.c_int]
     L.gl_stark_quotient.argtypes = [vp, vp, vp, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, C.c_uint32, vp]
+    L.gl_stark_quotient_aux.argtypes = [vp, vp, vp, vp, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, C.c_uint32, vp]
+    L.gl_stark_lookup_helper_columns.argtypes = [vp, vp, C.c_size_t, C.c_uint32, C.c_uint32, vp, vp, C.c_uint32, C.c_uint32,
+                                                 vp, C.c_int]
     L.gl_plonk_quotient.argtypes = [vp, vp, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, C.c_uint32,
                                     C.c_uint32, vp]
     L.gl_lookup_polys.argtypes = [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, vp, u32p, C.c_uint32, vp, C.c_int]

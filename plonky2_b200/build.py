@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libplonky2_b200.so")
 SOURCES = ["plonky2_b200.cu"]
-DEPS = ["plonky2_b200.cu", "gl_field.cuh", "gl_lazy.cuh", "gl_ntt.cuh", "gl_ntt_host.cuh", "gl_poseidon.cuh", "gl_poseidon_constants.h",
+DEPS = ["plonky2_b200.cu", "gl_field.cuh", "gl_logup.cuh", "gl_lazy.cuh", "gl_ntt.cuh", "gl_ntt_host.cuh", "gl_poseidon.cuh", "gl_poseidon_constants.h",
         os.path.join("..", "..", "include", "plonky2_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

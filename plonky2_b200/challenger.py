@@ -42,6 +42,12 @@ class Challenger:
         for h in cap.hashes:
             self.observe_hash(h)
 
+    def observe_openings(self, openings):
+        """observe_openings (plonky2/src/fri/challenges.rs:19-26): every batch's F_{p^2} values in order;
+        `openings` is a list of (k, 2) arrays (OpeningSet / StarkOpeningSet .to_fri_openings())."""
+        for batch in openings:
+            self.observe_elements([int(x) for x in batch.reshape(-1)])
+
     def get_challenge(self):
         if self.input_buffer or not self.output_buffer:
             self.duplexing()

@@ -23,6 +23,7 @@
 #include "gl_ntt.cuh"
 #include "gl_poseidon.cuh"
 #include "gl_vanishing.cuh"
+#include "gl_logup.cuh"
 
 using namespace gl;
 typedef uint64_t u64;
@@ -961,36 +962,46 @@ __global__ void __launch_bounds__(128) k_pp_chunks(PPParams p) {
         inv_run = mul(inv_run, den[m]);
     }
 }
-// multiplicative inclusive prefix scan, 3 phases
-__global__ void __launch_bounds__(SCAN_THREADS) k_mscan_phase1(const u64* seq, size_t L, u64* chunk_tot) {
+// inclusive prefix scan under a field operation (MulOp: partial products; AddOp: logUp Z), 3 phases
+struct MulOp {
+    static __device__ __forceinline__ u64 id() { return 1; }
+    static __device__ __forceinline__ u64 op(u64 a, u64 b) { return mul(a, b); }
+};
+struct AddOp {
+    static __device__ __forceinline__ u64 id() { return 0; }
+    static __device__ __forceinline__ u64 op(u64 a, u64 b) { return add(a, b); }
+};
+template <class Op>
+__global__ void __launch_bounds__(SCAN_THREADS) k_scan3_phase1(const u64* seq, size_t L, u64* chunk_tot) {
     __shared__ u64 sh[SCAN_THREADS];
     const size_t base = (size_t)blockIdx.x * SCAN_CHUNK + (size_t)threadIdx.x * SCAN_ITEMS;
-    u64 t = 1;
+    u64 t = Op::id();
     for (int k = 0; k < SCAN_ITEMS; k++)
-        if (base + k < L) t = mul(t, seq[base + k]);
+        if (base + k < L) t = Op::op(t, seq[base + k]);
     sh[threadIdx.x] = t;
     __syncthreads();
     for (int off = SCAN_THREADS / 2; off > 0; off >>= 1) {
-        if ((int)threadIdx.x < off) sh[threadIdx.x] = mul(sh[threadIdx.x], sh[threadIdx.x + off]);
+        if ((int)threadIdx.x < off) sh[threadIdx.x] = Op::op(sh[threadIdx.x], sh[threadIdx.x + off]);
         __syncthreads();
     }
     if (threadIdx.x == 0) chunk_tot[blockIdx.x] = sh[0];
 }
-// exclusive prefix products of the chunk totals, one CTA: each thread owns a contiguous run
-__global__ void __launch_bounds__(1024) k_mscan_phase2(u64* chunk_tot, size_t nchunks) {
+// exclusive prefix of the chunk totals, one CTA: each thread owns a contiguous run
+template <class Op>
+__global__ void __launch_bounds__(1024) k_scan3_phase2(u64* chunk_tot, size_t nchunks) {
     __shared__ u64 sh[1024];
     const size_t per = (nchunks + 1023) / 1024;
     const size_t lo = (size_t)threadIdx.x * per, hi = lo + per < nchunks ? lo + per : nchunks;
-    u64 t = 1;
-    for (size_t k = lo; k < hi; k++) t = mul(t, chunk_tot[k]);
+    u64 t = Op::id();
+    for (size_t k = lo; k < hi; k++) t = Op::op(t, chunk_tot[k]);
     sh[threadIdx.x] = t;
     __syncthreads();
-    if (threadIdx.x == 0) {  // 1024 sequential multiplies
-        u64 run = 1;
+    if (threadIdx.x == 0) {  // 1024 sequential steps
+        u64 run = Op::id();
         for (int k = 0; k < 1024; k++) {
             u64 v = sh[k];
             sh[k] = run;
-            run = mul(run, v);
+            run = Op::op(run, v);
         }
     }
     __syncthreads();
@@ -998,19 +1009,21 @@ __global__ void __launch_bounds__(1024) k_mscan_phase2(u64* chunk_tot, size_t nc
     for (size_t k = lo; k < hi; k++) {
         u64 v = chunk_tot[k];
         chunk_tot[k] = run;
-        run = mul(run, v);
+        run = Op::op(run, v);
     }
 }
-// phase 3: inclusive products inside each chunk; scatter to the output columns:
-// acc(i, m) -> partial product column m (m < M-1) at row i, or Z at row i+1 (m == M-1); Z(0) = 1.
-__global__ void __launch_bounds__(SCAN_THREADS) k_mscan_phase3(const u64* seq, size_t L, const u64* chunk_carry, size_t n,
+// phase 3: inclusive prefix inside each chunk; scatter to the output columns:
+// acc(i, m) -> partial product column m (m < M-1) at row i, or Z at row i+1 (m == M-1); Z(0) = the identity.
+// With M = 1 this is the exclusive scan of one column into out (seq and out must not overlap).
+template <class Op>
+__global__ void __launch_bounds__(SCAN_THREADS) k_scan3_phase3(const u64* seq, size_t L, const u64* chunk_carry, size_t n,
                                                              uint32_t M, u64* out) {
     __shared__ u64 sh[SCAN_THREADS];
     const size_t base = (size_t)blockIdx.x * SCAN_CHUNK + (size_t)threadIdx.x * SCAN_ITEMS;
     u64 loc[SCAN_ITEMS];
-    u64 run = 1;
+    u64 run = Op::id();
     for (int k = 0; k < SCAN_ITEMS; k++) {
-        if (base + k < L) run = mul(run, seq[base + k]);
+        if (base + k < L) run = Op::op(run, seq[base + k]);
         loc[k] = run;
     }
     sh[threadIdx.x] = run;
@@ -1020,7 +1033,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_mscan_phase3(const u64* seq, s
         for (int t = 0; t < SCAN_THREADS; t++) {
             u64 v = sh[t];
             sh[t] = r;
-            r = mul(r, v);
+            r = Op::op(r, v);
         }
     }
     __syncthreads();
@@ -1028,12 +1041,12 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_mscan_phase3(const u64* seq, s
     for (int k = 0; k < SCAN_ITEMS; k++) {
         const size_t t = base + k;
         if (t >= L) break;
-        const u64 acc = canon(mul(carry, loc[k]));
+        const u64 acc = canon(Op::op(carry, loc[k]));
         const size_t i = t / M, m = t % M;
         if (m + 1 < M) out[m * n + i] = acc;
         else if (i + 1 < n) out[(size_t)(M - 1) * n + i + 1] = acc;
     }
-    if (blockIdx.x == 0 && threadIdx.x == 0) out[(size_t)(M - 1) * n] = 1;
+    if (blockIdx.x == 0 && threadIdx.x == 0) out[(size_t)(M - 1) * n] = Op::id();
 }
 
 // ---- lookup argument helper columns (compute_lookup_polys, plonk/prover.rs:458-577; SURVEY 8(f) row 3) ----
@@ -1138,6 +1151,8 @@ __global__ void __launch_bounds__(1024) k_affine_scan(const u64* b, size_t len, 
 struct StarkQuotientParams {
     const u64* lde;        // trace LDE, column k at lde + k*lde_stride, leaf order
     size_t lde_stride;
+    const u64* aux;        // auxiliary polynomials' LDE (same degree and rate, same layout), or null
+    size_t aux_stride;
     uint32_t log_N;        // log2 of the LDE size
     uint32_t degree_bits, qd_bits;
     const gl_stark_instr* prog;
@@ -1182,6 +1197,8 @@ __global__ void __launch_bounds__(128) k_stark_quotient(StarkQuotientParams p) {
         switch (in.op) {
             case GL_STARK_LOCAL: r = p.lde[(size_t)in.a * p.lde_stride + jl]; break;
             case GL_STARK_NEXT: r = p.lde[(size_t)in.a * p.lde_stride + jn]; break;
+            case GL_STARK_AUX_LOCAL: r = p.aux[(size_t)in.a * p.aux_stride + jl]; break;
+            case GL_STARK_AUX_NEXT: r = p.aux[(size_t)in.a * p.aux_stride + jn]; break;
             case GL_STARK_CONST: r = p.consts[in.a]; break;
             case GL_STARK_ADD: r = add(v[in.a], v[in.b]); break;
             case GL_STARK_SUB: r = sub(v[in.a], v[in.b]); break;
@@ -1198,6 +1215,14 @@ __global__ void __launch_bounds__(128) k_stark_quotient(StarkQuotientParams p) {
     }
     const u64 zi = p.zh_inv[i & (((size_t)1 << p.qd_bits) - 1)];
     for (uint32_t a = 0; a < p.n_alphas; a++) p.out[(size_t)a * size + i] = canon(mul(acc[a], zi));
+}
+// ---- starky logUp helper columns (lookup_helper_columns, starky/src/lookup.rs:579-652): one thread per trace row; the
+// row's evaluation is gl_logup.cuh, the Z columns are the exclusive additive scan (k_scan3_*<AddOp>) of its terms
+__global__ void __launch_bounds__(128) k_logup_rows(LogupParams p, unsigned int* flag) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= p.n) return;
+    u64 den[GL_LOGUP_MAX_DENOMINATORS], pre[GL_LOGUP_MAX_DENOMINATORS];
+    if (!logup_eval_row(p, i, den, pre)) atomicOr(flag, 1u);
 }
 // any non-zero word in [begin, begin + count) of each of `cols` columns (stride `stride`) -> flag
 __global__ void k_any_nonzero(const u64* data, size_t stride, size_t begin, size_t count, unsigned int* flag) {
@@ -1770,11 +1795,11 @@ int gl_partial_products_and_zs(gl_ctx* ctx, const uint64_t* wires, const uint64_
                     (unsigned int*)dflag};
         k_pp_chunks<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(pp);
         CKL(ctx);
-        k_mscan_phase1<<<(unsigned)nchunks, SCAN_THREADS, 0, ctx->stream>>>(seq, L, tot);
+        k_scan3_phase1<MulOp><<<(unsigned)nchunks, SCAN_THREADS, 0, ctx->stream>>>(seq, L, tot);
         CKL(ctx);
-        k_mscan_phase2<<<1, 1024, 0, ctx->stream>>>(tot, nchunks);
+        k_scan3_phase2<MulOp><<<1, 1024, 0, ctx->stream>>>(tot, nchunks);
         CKL(ctx);
-        k_mscan_phase3<<<(unsigned)nchunks, SCAN_THREADS, 0, ctx->stream>>>(seq, L, tot, n, M, dout);
+        k_scan3_phase3<MulOp><<<(unsigned)nchunks, SCAN_THREADS, 0, ctx->stream>>>(seq, L, tot, n, M, dout);
         CKL(ctx);
         u64 flag = 0;
         TRY(d2h(ctx, &flag, dflag, 1));
@@ -1884,12 +1909,26 @@ int gl_lookup_polys(gl_ctx* ctx, const uint64_t* wires, uint32_t log_n, uint32_t
 int gl_stark_quotient(gl_ctx* ctx, gl_commit* trace, const gl_stark_instr* program, uint32_t n_instr,
                       const uint64_t* consts, uint32_t n_consts, const uint64_t* alphas, uint32_t n_alphas,
                       uint32_t quotient_degree_factor, uint64_t* out_coeffs) {
+    return gl_stark_quotient_aux(ctx, trace, nullptr, program, n_instr, consts, n_consts, alphas, n_alphas,
+                                 quotient_degree_factor, out_coeffs);
+}
+
+int gl_stark_quotient_aux(gl_ctx* ctx, gl_commit* trace, gl_commit* aux, const gl_stark_instr* program, uint32_t n_instr,
+                          const uint64_t* consts, uint32_t n_consts, const uint64_t* alphas, uint32_t n_alphas,
+                          uint32_t quotient_degree_factor, uint64_t* out_coeffs) {
     if (!ctx || !trace || !program || !alphas || !out_coeffs) return set_err(ctx, GL_ERR_BAD_ARG, "null argument");
     if (n_instr == 0 || n_instr > GL_STARK_MAX_INSTR) return set_err(ctx, GL_ERR_UNSUPPORTED, "program of %u instructions (max %d)", n_instr, GL_STARK_MAX_INSTR);
     if (n_alphas == 0 || n_alphas > GL_STARK_MAX_ALPHAS) return set_err(ctx, GL_ERR_UNSUPPORTED, "1..%d challenges", GL_STARK_MAX_ALPHAS);
     if (quotient_degree_factor == 0) return set_err(ctx, GL_ERR_BAD_ARG, "quotient_degree_factor is 0: the STARK has no quotient");
     if (trace->shard_log) return set_err(ctx, GL_ERR_UNSUPPORTED, "quotient evaluation needs the whole LDE on this device");
     NEED_FINISHED(trace);
+    if (aux) {
+        NEED_FINISHED(aux);
+        if (aux->shard_log) return set_err(ctx, GL_ERR_UNSUPPORTED, "quotient evaluation needs the whole LDE on this device");
+        if (aux->degree_log != trace->degree_log || aux->rate_bits != trace->rate_bits)
+            return set_err(ctx, GL_ERR_BAD_SHAPE, "auxiliary polynomials of degree 2^%u rate_bits %u, trace 2^%u rate_bits %u",
+                           aux->degree_log, aux->rate_bits, trace->degree_log, trace->rate_bits);
+    }
     uint32_t qd_bits = 0;
     while ((1u << qd_bits) < quotient_degree_factor) qd_bits++;  // log2_ceil
     if (qd_bits > trace->rate_bits)
@@ -1900,6 +1939,7 @@ int gl_stark_quotient(gl_ctx* ctx, gl_commit* trace, const gl_stark_instr* progr
         bool ok = true;
         switch (in.op) {
             case GL_STARK_LOCAL: case GL_STARK_NEXT: ok = in.a < trace->B; break;
+            case GL_STARK_AUX_LOCAL: case GL_STARK_AUX_NEXT: ok = aux && in.a < aux->B; break;
             case GL_STARK_CONST: ok = in.a < n_consts; break;
             case GL_STARK_ADD: case GL_STARK_SUB: case GL_STARK_MUL: ok = in.a < k && in.b < k; break;
             case GL_STARK_EMIT: ok = in.a < k && in.b <= GL_STARK_LAST_ROW; break;
@@ -1925,6 +1965,8 @@ int gl_stark_quotient(gl_ctx* ctx, gl_commit* trace, const gl_stark_instr* progr
         StarkQuotientParams p;
         p.lde = trace->tree.leaves;
         p.lde_stride = trace->tree.es;
+        p.aux = aux ? aux->tree.leaves : nullptr;
+        p.aux_stride = aux ? aux->tree.es : 0;
         p.log_N = db + trace->rate_bits;
         p.degree_bits = db;
         p.qd_bits = qd_bits;
@@ -1971,6 +2013,127 @@ int gl_stark_quotient(gl_ctx* ctx, gl_commit* trace, const gl_stark_instr* progr
     dfree(ctx, dconst);
     dfree(ctx, xtab);
     dfree(ctx, dflag);
+    return rc;
+}
+
+int gl_stark_lookup_helper_columns(gl_ctx* ctx, const uint64_t* trace, size_t col_stride, uint32_t n_cols, uint32_t log_n,
+                                   const gl_logup_desc* desc, const uint64_t* challenges, uint32_t n_challenges,
+                                   uint32_t constraint_degree, uint64_t* out, int mem) {
+    if (!ctx || !trace || !desc || !out || (n_challenges && !challenges)) return set_err(ctx, GL_ERR_BAD_ARG, "null argument");
+    if (mem != GL_MEM_HOST && mem != GL_MEM_DEVICE) return set_err(ctx, GL_ERR_BAD_ARG, "bad mem %d", mem);
+    if (log_n > 30) return set_err(ctx, GL_ERR_UNSUPPORTED, "log_n %u > 30", log_n);
+    const size_t n = (size_t)1 << log_n;
+    if (col_stride < n) return set_err(ctx, GL_ERR_BAD_SHAPE, "col_stride %zu < n = %zu", col_stride, n);
+    const gl_logup_desc& d = *desc;
+    if ((d.n_terms && !d.terms) || (d.n_columns && (!d.columns || !d.filters)) || (d.n_filter_columns && !d.filter_columns) ||
+        (d.n_lookups && !d.lookups))
+        return set_err(ctx, GL_ERR_BAD_ARG, "null descriptor array");
+    // validate once on the host: the kernel trusts the descriptors
+    for (uint32_t t = 0; t < d.n_terms; t++)
+        if (d.terms[t].col >= n_cols || d.terms[t].next > 1) return set_err(ctx, GL_ERR_BAD_ARG, "lookup term %u: bad column", t);
+    for (uint32_t c = 0; c < d.n_columns; c++) {
+        const gl_logup_filter f = d.filters[c];
+        if ((uint64_t)d.columns[c].term_begin + d.columns[c].n_terms > d.n_terms ||
+            (uint64_t)f.prod_begin + 2 * (uint64_t)f.n_prods > d.n_filter_columns ||
+            (uint64_t)f.sum_begin + f.n_sums > d.n_filter_columns)
+            return set_err(ctx, GL_ERR_BAD_ARG, "lookup column %u: range outside the descriptor arrays", c);
+    }
+    for (uint32_t k = 0; k < d.n_filter_columns; k++)
+        if (d.filter_columns[k] >= d.n_columns) return set_err(ctx, GL_ERR_BAD_ARG, "filter column %u: bad index", k);
+    const uint32_t chunk = constraint_degree > 2 ? constraint_degree - 1 : 1;  // constraint_degree.checked_sub(1), at least 1
+    uint64_t n_den = 0, n_out = 0;
+    std::vector<uint32_t> zcols;  // output column of every (lookup, challenge) Z
+    for (uint32_t l = 0; l < d.n_lookups; l++) {
+        const gl_logup_lookup lk = d.lookups[l];
+        if ((uint64_t)lk.looking_begin + lk.n_looking > d.n_columns || lk.table >= d.n_columns || lk.frequencies >= d.n_columns)
+            return set_err(ctx, GL_ERR_BAD_ARG, "lookup %u: bad column index", l);
+        n_den += (uint64_t)(lk.n_looking + 1) * n_challenges;
+        const uint32_t nh = (lk.n_looking + chunk - 1) / chunk + 1;  // Lookup::num_helper_columns
+        for (uint32_t c = 0; c < n_challenges; c++) {
+            n_out += nh;
+            zcols.push_back((uint32_t)n_out - 1);
+        }
+    }
+    if (n_den > GL_LOGUP_MAX_DENOMINATORS)
+        return set_err(ctx, GL_ERR_UNSUPPORTED, "%llu denominators per row (max %d)", (unsigned long long)n_den,
+                       GL_LOGUP_MAX_DENOMINATORS);
+    if (zcols.empty()) return GL_OK;
+    CK(ctx, cudaSetDevice(ctx->device));
+    u64 *ddesc = nullptr, *dchal = nullptr, *dtrace = nullptr, *dout = nullptr, *zterm = nullptr, *tot = nullptr, *dflag = nullptr;
+    auto body = [&]() -> int {
+        // the descriptor arrays, packed into one device buffer
+        const size_t sz[5] = {d.n_terms * sizeof(gl_logup_term), d.n_columns * sizeof(gl_logup_column),
+                              d.n_columns * sizeof(gl_logup_filter), d.n_lookups * sizeof(gl_logup_lookup),
+                              d.n_filter_columns * sizeof(uint32_t)};
+        const void* src[5] = {d.terms, d.columns, d.filters, d.lookups, d.filter_columns};
+        size_t off[5], words = 0;
+        for (int k = 0; k < 5; k++) {
+            off[k] = words;
+            words += (sz[k] + 15) / 16 * 2;
+        }
+        TRY(dmalloc(ctx, &ddesc, words ? words : 1));
+        for (int k = 0; k < 5; k++)
+            if (sz[k]) CK(ctx, cudaMemcpyAsync(ddesc + off[k], src[k], sz[k], cudaMemcpyHostToDevice, ctx->stream));
+        TRY(dmalloc(ctx, &dchal, n_challenges));
+        std::vector<u64> ch(n_challenges);
+        for (uint32_t c = 0; c < n_challenges; c++) ch[c] = canon(challenges[c]);
+        TRY(h2d(ctx, dchal, ch.data(), n_challenges));
+        LogupParams p;
+        p.d = d;
+        p.d.terms = (const gl_logup_term*)(ddesc + off[0]);
+        p.d.columns = (const gl_logup_column*)(ddesc + off[1]);
+        p.d.filters = (const gl_logup_filter*)(ddesc + off[2]);
+        p.d.lookups = (const gl_logup_lookup*)(ddesc + off[3]);
+        p.d.filter_columns = (const uint32_t*)(ddesc + off[4]);
+        if (mem == GL_MEM_HOST) {
+            TRY(dmalloc(ctx, &dtrace, (size_t)n_cols * n ? (size_t)n_cols * n : 1));
+            if (n_cols)
+                CK(ctx, cudaMemcpy2DAsync(dtrace, n * 8, trace, col_stride * 8, n * 8, n_cols, cudaMemcpyHostToDevice, ctx->stream));
+            p.trace = dtrace;
+            p.col_stride = n;
+            TRY(dmalloc(ctx, &dout, n_out * n));
+        } else {
+            p.trace = trace;
+            p.col_stride = col_stride;
+            dout = out;
+        }
+        p.n = n;
+        p.challenges = dchal;
+        p.n_challenges = n_challenges;
+        p.chunk = chunk;
+        p.out = dout;
+        TRY(dmalloc(ctx, &zterm, zcols.size() * n));
+        p.zterm = zterm;
+        TRY(dmalloc(ctx, &dflag, 1));
+        CK(ctx, cudaMemsetAsync(dflag, 0, 8, ctx->stream));
+        k_logup_rows<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(p, (unsigned int*)dflag);
+        CKL(ctx);
+        // Z(0) = 0, Z(i+1) = Z(i) + d(i): exclusive scan of every Z's terms into its column
+        const size_t nchunks = (n + SCAN_CHUNK - 1) / SCAN_CHUNK;
+        TRY(dmalloc(ctx, &tot, nchunks));
+        for (size_t z = 0; z < zcols.size(); z++) {
+            const u64* seq = zterm + z * n;
+            k_scan3_phase1<AddOp><<<(unsigned)nchunks, SCAN_THREADS, 0, ctx->stream>>>(seq, n, tot);
+            CKL(ctx);
+            k_scan3_phase2<AddOp><<<1, 1024, 0, ctx->stream>>>(tot, nchunks);
+            CKL(ctx);
+            k_scan3_phase3<AddOp><<<(unsigned)nchunks, SCAN_THREADS, 0, ctx->stream>>>(seq, n, tot, n, 1, dout + (size_t)zcols[z] * n);
+            CKL(ctx);
+        }
+        u64 flag = 0;
+        TRY(d2h(ctx, &flag, dflag, 1));
+        if (flag & 1u) return set_err(ctx, GL_ERR_DIV_ZERO, "Tried to invert zero");
+        if (mem == GL_MEM_HOST) TRY(d2h(ctx, out, dout, n_out * n));
+        return GL_OK;
+    };
+    int rc = body();
+    dfree(ctx, ddesc);
+    dfree(ctx, dchal);
+    dfree(ctx, dtrace);
+    dfree(ctx, zterm);
+    dfree(ctx, tot);
+    dfree(ctx, dflag);
+    if (mem == GL_MEM_HOST) dfree(ctx, dout);
     return rc;
 }
 

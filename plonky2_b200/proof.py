@@ -115,3 +115,22 @@ class StarkOpeningSet:
             zeta_batch.append(self.quotient_polys)
         next_batch = [self.next_values] + ([self.auxiliary_polys_next] if self.auxiliary_polys_next is not None else [])
         return [np.concatenate(zeta_batch), np.concatenate(next_batch)]
+
+
+@dataclass
+class StarkProof:
+    """StarkProof<F, C, D> (starky/src/proof.rs:27-40) without cross-table lookups. The caps are MerkleCaps (None where
+    the STARK has no auxiliary or no quotient polynomials); opening_proof is a FriProof, whose to_bytes() is
+    write_fri_proof. The reference serialises a STARK proof with serde only, so there is no byte format here."""
+    trace_cap: object
+    auxiliary_polys_cap: object
+    quotient_polys_cap: object
+    openings: StarkOpeningSet
+    opening_proof: object
+
+
+@dataclass
+class StarkProofWithPublicInputs:
+    """StarkProofWithPublicInputs (starky/src/proof.rs:150-158)."""
+    proof: StarkProof
+    public_inputs: list
